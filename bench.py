@@ -2,7 +2,7 @@
 """bench.py — waveforms/s of the seist_m_dpk training step (fwd + BCE + bwd + Adam) on (B,3,8192)
 synthetic seismograms; see DESIGN.md §5 for what each JSON key means.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 """
 import argparse
@@ -133,6 +133,32 @@ def reference_step_rate(model_name, batch, length, steps, warmup, threads, devic
     return batch * len(times) / sum(times), sum(times), kind
 
 
+DUMP_BYTES = 60 << 20      # bound on the arrays of one --dump-outputs directory (under 64 MB with the file headers)
+DUMP_ROWS = 64             # waveforms of the predictions kept in a dump, a fixed seeded sample of the batch
+
+
+def dump_outputs(out_dir, trainer):
+    """Writes what the last Trainer.step() computed, as its caller sees it, to out_dir/<name>.npy (float32): the loss,
+    the model's predictions (rows listed in prediction_rows.npy), the parameter gradients, and the parameters and
+    BatchNorm running statistics after the Adam update.  Two builds run with the same arguments can be compared
+    array by array."""
+    import numpy as np
+    y = trainer.plan.y_out.x
+    arrays = {"loss": trainer.loss_out, "gradients": trainer.last_grads, "parameters": trainer.flat.P,
+              "bn_running_stats": trainer.flat.RB}
+    row_bytes = y[0].numel() * 4
+    budget = DUMP_BYTES - sum(t.numel() * 4 for t in arrays.values())
+    n = min(y.shape[0], DUMP_ROWS, budget // row_bytes)
+    if n < 1:
+        raise ValueError(f"--dump-outputs: the outputs of one step exceed {DUMP_BYTES >> 20} MB")
+    rows = torch.randperm(y.shape[0], generator=torch.Generator().manual_seed(0))[:n].sort().values
+    arrays["predictions"] = y[rows.to(y.device)]
+    arrays["prediction_rows"] = rows
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().to("cpu", torch.float32).numpy())
+
+
 def _kind_text(kind):
     return ("unmodified reference modules staged in oracle/_ref, default drop rates" if kind == "reference"
             else "oracle port of the reference step, dropout identity")
@@ -161,7 +187,13 @@ def main():
     ap.add_argument("--cpu-batch", type=int, default=32)
     ap.add_argument("--cpu-steps", type=int, default=12)
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy (float32, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs needs --impl native")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -176,7 +208,7 @@ def main():
     if args.impl == "reference":
         if rank != 0:
             return
-        steps = max(1, min(args.steps, 20))      # bounded sample: ~0.5 s per 32-waveform CPU step
+        steps = args.steps                       # ~0.5 s per 32-waveform CPU step
         warm = max(1, min(args.warmup, 2))
         rate, secs, kind = reference_step_rate(args.model, args.cpu_batch, args.length, steps, warm, cores)
         config["cpu_sample_batch"] = args.cpu_batch
@@ -250,6 +282,8 @@ def main():
     if profiling:
         torch.cuda.profiler.stop()
     clocks = sampler.summary(t0, t1) if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, trainer)
     loss_val = float(trainer.loss_out.item())
     value = args.batch * world * args.steps / (ms / 1e3)
 

@@ -1,4 +1,4 @@
-"""Generate tests/golden/*.pt by executing the UNMODIFIED reference (/root/reference).
+"""Generate the tests/golden/<model>.<i>.pt fixtures (oracle/fixtures.py) by executing the UNMODIFIED reference.
 
 Run in the build container only:  python tests/golden/make_golden.py
 Each fixture holds: the reference's pretrained state_dict (weights are the only pinned artefacts the
@@ -14,6 +14,7 @@ import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
+from oracle import fixtures  # noqa: E402
 from oracle import reference_import as ri  # noqa: E402
 from oracle import seist_ref as R  # noqa: E402
 
@@ -66,9 +67,8 @@ def main():
             "grads": {k: p.grad.clone() for k, p in model.named_parameters()},
             "buffers_after": {k: b.clone() for k, b in model.named_buffers()},
         }
-        path = os.path.join(HERE, f"{name}.pt")
-        torch.save(out, path)
-        print(name, "->", path, os.path.getsize(path) // 1024, "KiB", "loss", float(loss))
+        fixtures.save(out, HERE, name)
+        print(name, "->", HERE, "loss", float(loss))
 
 
 if __name__ == "__main__":

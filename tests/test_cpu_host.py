@@ -6,6 +6,7 @@ import os
 import pytest
 import torch
 
+from oracle import fixtures
 from oracle import seist_ref as R
 from oracle.plan_interp import Interp, keep_mask, rng_u16
 from seist_b200 import _lib
@@ -34,7 +35,7 @@ def test_registry_surface():
 
 @pytest.mark.parametrize("name", ["seist_s_dpk", "seist_m_dpk", "seist_m_emg"])
 def test_state_dict_matches_reference_checkpoint(name):
-    g = torch.load(os.path.join(GOLD, f"{name}.pt"))
+    g = fixtures.load(GOLD, name)
     m = create_model(name, in_channels=3, in_samples=8192)
     sd = m.state_dict()
     assert list(sd.keys()) == list(g["state_dict"].keys())
@@ -67,7 +68,7 @@ def test_channel_arithmetic():
 def test_plan_compiler_end_to_end_vs_reference_golden():
     """Forward tape, derived backward, accumulate flags and the BN-backward algebra, executed by the CPU
     interpreter, reproduce the reference's outputs, gradients and running statistics."""
-    g = torch.load(os.path.join(GOLD, "seist_s_dpk.pt"))
+    g = fixtures.load(GOLD, "seist_s_dpk")
     m = create_model("seist_s_dpk", in_channels=3, in_samples=8192)
     m.load_state_dict(g["state_dict"], strict=True)
     m.set_drop_rates(**ZERO)
@@ -98,7 +99,7 @@ def test_plan_compiler_end_to_end_vs_reference_golden():
 
 def test_plan_compiler_regression_head_vs_reference_golden():
     """Same as above for the regression family (seist_m_emg: HEADVEC ops, scaled sigmoid, Huber loss)."""
-    g = torch.load(os.path.join(GOLD, "seist_m_emg.pt"))
+    g = fixtures.load(GOLD, "seist_m_emg")
     m = create_model("seist_m_emg", in_channels=3, in_samples=8192)
     m.load_state_dict(g["state_dict"], strict=True)
     m.set_drop_rates(**ZERO)
@@ -162,7 +163,7 @@ def test_grad_combine_plan_equals_default_plan(monkeypatch):
     """GRAD_COMBINE (opt-in, SEIST_COMBINE_CIN): the compiler marks the wide 1x1 convs, emits the in-place BN
     backward before their three backward ops and re-points those ops at the combined gradient; executed by the
     interpreter the parameter gradients must equal the default plan's (reference golden batch, train mode)."""
-    g = torch.load(os.path.join(GOLD, "seist_s_dpk.pt"))
+    g = fixtures.load(GOLD, "seist_s_dpk")
     x = g["x"][:2, :, :2048].contiguous()
     tgt = g["target"][:2, :, :2048].contiguous()
 

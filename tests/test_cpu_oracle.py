@@ -1,19 +1,23 @@
-"""not-gpu: the oracle restatement against the golden vectors produced by the unmodified reference, and
-(in the build container, where /root/reference exists) against the reference's own modules."""
+"""not-gpu: the oracle restatement against the golden vectors produced by the unmodified reference, and against
+stored results of the reference's own modules (tests/golden/make_reference_checks.py)."""
+import json
 import os
 
+import numpy as np
 import pytest
 import torch
 
-from oracle import reference_import as ri
+import reference_inputs as I
+from oracle import fixtures
 from oracle import seist_ref as R
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+REF = np.load(os.path.join(GOLD, "reference_checks.npz"))
 
 
 @pytest.mark.parametrize("name", ["seist_s_dpk", "seist_m_dpk", "seist_m_emg", "seist_s_pmp", "seist_s_baz"])
 def test_oracle_matches_golden(name):
-    g = torch.load(os.path.join(GOLD, f"{name}.pt"))
+    g = fixtures.load(GOLD, name)
     spec = R.spec_for(name)
     with torch.no_grad():
         y, _ = R.forward(g["state_dict"], g["x"], spec, training=False)
@@ -33,19 +37,13 @@ def test_oracle_matches_golden(name):
         assert (bufs[k].float() - b.float()).abs().max().item() <= 1e-5 * (b.float().abs().max().item() + 1e-3), k
 
 
-@pytest.mark.skipif(not ri.available(), reason="reference checkout not present (GPU box)")
 def test_oracle_matches_reference_modules():
-    M = ri.import_reference_models()
-    torch.manual_seed(0)
-    for name in ("seist_s_dpk", "seist_l_emg", "seist_s_pmp"):
-        ref = ri.zero_drop_rates(M.create_model(name, in_channels=3, in_samples=2048))
-        with torch.no_grad():   # de-generate the init a little so the comparison is meaningful
-            for p in ref.parameters():
-                p.add_(0.05 * torch.randn_like(p))
-        x = torch.randn(2, 3, 2048)
-        ref.train()
-        y_ref = ref(x)
-        y, _ = R.forward(ref.state_dict(), x, R.spec_for(name), training=True)
+    """Train mode, drop rates zeroed: the oracle against the output of the reference's modules on the same parameters."""
+    for name in I.MODULE_MODELS:
+        sd, x = I.module_inputs(name)
+        assert np.array_equal(I.probe(x.numpy()), REF[f"modules.{name}.x_probe"]), "seeded input changed"
+        y_ref = torch.from_numpy(REF[f"modules.{name}.y"])
+        y, _ = R.forward(sd, x, R.spec_for(name), training=True)
         assert torch.allclose(y, y_ref, atol=1e-6), name
 
 
@@ -65,8 +63,7 @@ def test_pad_and_sizes():
                                                          (16, 16, 7), (16, 6, 11)]
 
 
-@pytest.mark.skipif(not ri.available(), reason="reference checkout not present (GPU box)")
-@pytest.mark.parametrize("name", ["seist_s_dpk", "seist_m_dpk", "seist_l_dpk", "seist_m_emg"])
+@pytest.mark.parametrize("name", I.DROPOUT_MODELS)
 def test_dropout_sites_and_rates_match_reference_modules(name):
     """Every nn.Dropout / timm DropPath of the unmodified reference model (site = module path, rate = .p / .drop_prob,
     models/seist.py:114,228,239,360-366,446,470,484; linspace schedule :705) must appear in the compiled plan as the
@@ -74,17 +71,10 @@ def test_dropout_sites_and_rates_match_reference_modules(name):
     from seist_b200 import _lib
     from seist_b200 import plan as P
     from seist_b200.models import create_model
-    M = ri.import_reference_models()
-    ref = M.create_model(name, in_channels=3, in_samples=1024)
+    with open(os.path.join(GOLD, "reference_dropout_sites.json")) as f:
+        ref_sites = json.load(f)[name]          # [module path, rate] of the reference model's modules
     expect = {}
-    for path, mod in ref.named_modules():
-        cls = mod.__class__.__name__
-        if cls == "Dropout":
-            p = float(mod.p)
-        elif cls == "DropPath":
-            p = float(mod.drop_prob or 0.0)
-        else:
-            continue
+    for path, p in ref_sites:
         head, leaf = path.rsplit(".", 1)
         site = {
             "droppath0": (head + ".proj", "p_path"),

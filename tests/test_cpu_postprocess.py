@@ -1,53 +1,25 @@
-"""not-gpu: the post-processing oracle (oracle/postprocess_ref.py) against the reference's own `_detect_peaks`, executed
-from its source (the module itself needs obspy / pandas, which are absent; the function only needs numpy)."""
-import ast
+"""not-gpu: the post-processing oracle (oracle/postprocess_ref.py) against the picks of the reference's own
+`_detect_peaks`, stored in tests/golden/reference_checks.npz (tests/golden/make_reference_checks.py)."""
 import os
 
 import numpy as np
 import pytest
 
+import reference_inputs as I
 from oracle import postprocess_ref as PR
-from oracle import reference_import as ri
+
+REF = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_checks.npz"))
 
 
-def _reference_detect_peaks():
-    path = os.path.join(ri.REF_ROOT, "training", "postprocess.py")
-    tree = ast.parse(open(path).read())
-    fn = next(n for n in tree.body if isinstance(n, ast.FunctionDef) and n.name == "_detect_peaks")
-    ns = {"np": np}
-    exec(compile(ast.Module(body=[fn], type_ignores=[]), path, "exec"), ns)      # noqa: S102 - the reference's own code
-    return ns["_detect_peaks"]
-
-
-def _traces(rng, n, L):
-    t = np.arange(L, dtype=np.float32)
-    out = np.zeros((n, L), dtype=np.float32)
-    for i in range(n):
-        for _ in range(rng.integers(0, 6)):
-            c, w, a = rng.integers(0, L), rng.uniform(3, 40), rng.uniform(0.1, 1.0)
-            out[i] += a * np.exp(-((t - c) ** 2) / (2 * w * w)).astype(np.float32)
-        out[i] = out[i] + 0.02 * rng.standard_normal(L).astype(np.float32)
-        # no clipping: equal peak heights have no defined order in the reference (np.argsort's default sort is unstable)
-        out[i] = (out[i] - out[i].min()) / max(1.0, float(out[i].max() - out[i].min()) * 1.01)
-    return out
-
-
-@pytest.mark.skipif(not ri.available(), reason="reference checkout not present (GPU box)")
-@pytest.mark.parametrize("topk,mpd", [(1, 50), (3, 50), (5, 8), (2, 200)])
+@pytest.mark.parametrize("topk,mpd", I.PICK_CASES)
 def test_pick_phase_matches_reference_detect_peaks(topk, mpd):
-    ref = _reference_detect_peaks()
-    rng = np.random.default_rng(topk * 100 + mpd)
-    x = _traces(rng, 48, 2048)
-    x[0] = 0.0                          # no peak at all
-    x[1, :] = 0.5                       # flat above the threshold: no rising edge
-    x[2] = 0.0
-    x[2, 100:110] = 0.8                 # flat-topped peak: rising edge only
-    x[3] = 0.0
-    x[3, 0], x[3, -1] = 0.9, 0.9        # first / last samples cannot be peaks
-    for thr in (0.3, 0.05):
+    x = I.pick_traces(topk, mpd)
+    assert np.array_equal(I.probe(x), REF[f"pick.{topk}_{mpd}.x_probe"]), "seeded input changed"
+    for thr in I.PICK_THRESHOLDS:
         mine = PR.pick_phase(x, thr, mpd, topk)
-        for i, row in enumerate(x):
-            want = ref(row, mph=thr, mpd=mpd, topk=topk)
+        ref = REF[f"pick.{topk}_{mpd}.{thr}"]
+        for i in range(x.shape[0]):
+            want = ref[i][ref[i] != PR.PAD_PHASE]
             got = mine[i][mine[i] != PR.PAD_PHASE]
             assert np.array_equal(got, want), (i, thr, got, want)
             assert (mine[i][got.size:] == PR.PAD_PHASE).all()

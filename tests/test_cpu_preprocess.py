@@ -1,46 +1,22 @@
-"""not-gpu: the input-side oracle (oracle/preprocess_ref.py) against the reference's own `_normalize`, `_pad_phases` and
-`_generate_soft_label`, executed from their sources (training/preprocess.py imports h5py-backed datasets, absent here)."""
-import ast
+"""not-gpu: the input-side oracle (oracle/preprocess_ref.py) against the results of the reference's own `_normalize`,
+`_pad_phases` and `_generate_soft_label`, stored in tests/golden/reference_checks.npz
+(tests/golden/make_reference_checks.py)."""
 import os
-from types import SimpleNamespace
-from typing import Any, List, Tuple, Union
 
 import numpy as np
-import pytest
 
+import reference_inputs as I
 from oracle import preprocess_ref as PR
-from oracle import reference_import as ri
+
+REF = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_checks.npz"))
 
 
-def _reference_functions():
-    path = os.path.join(ri.REF_ROOT, "training", "preprocess.py")
-    tree = ast.parse(open(path).read())
-    ns = {"np": np, "Tuple": Tuple, "Union": Union, "List": List, "Any": Any}
-    body = [n for n in tree.body if isinstance(n, ast.FunctionDef) and n.name == "_pad_phases"]
-    cls = next(n for n in tree.body if isinstance(n, ast.ClassDef) and n.name == "DataPreprocessor")
-    body += [n for n in cls.body if isinstance(n, ast.FunctionDef) and n.name in ("_normalize", "_generate_soft_label")]
-    exec(compile(ast.Module(body=body, type_ignores=[]), path, "exec"), ns)      # noqa: S102 - the reference's own code
-    return ns
-
-
-@pytest.mark.skipif(not ri.available(), reason="reference checkout not present (GPU box)")
 def test_input_side_oracle_matches_reference_sources():
-    ns = _reference_functions()
-    rng = np.random.default_rng(0)
-    for mode in ("std", "max", ""):
-        x = rng.standard_normal((3, 4096)).astype(np.float32) * 3 + 1
-        x[1] = 2.5                                                   # constant channel: scale 0 -> 1
-        want = ns["_normalize"](None, x.copy(), mode)
+    for mode, x in I.normalize_inputs():
+        want = REF[f"normalize.{mode or 'none'}"]
         assert np.array_equal(PR.normalize(x, mode), want), mode
-    L = 2048
-    me = SimpleNamespace(coda_ratio=1.4, dtype=np.float32, data_channels=["z", "n", "e"])
-    cases = [([300], [700]), ([5], [60]), ([1900], [2040]), ([], []), ([100, 900], [400, 1300]), ([800], []), ([], [500]),
-             ([2047], [2047 + 30]), ([0], [3])]
-    for shape in ("gaussian", "triangle", "box"):
-        for width in (25, 50, 11):
-            for ppks, spks in cases:
-                ev = {"data": np.zeros((3, L), np.float32), "ppks": list(ppks), "spks": list(spks)}
-                got = PR.dpk_labels(ppks, spks, L, width, shape, 1.4)
-                for row, name in enumerate(("det", "ppk", "spk")):
-                    want = ns["_generate_soft_label"](me, name, ev, width, shape)
-                    assert np.array_equal(got[row], want), (shape, width, ppks, spks, name)
+    for shape, width, ci, ppks, spks in I.label_cases():
+        got = PR.dpk_labels(ppks, spks, I.LABEL_L, width, shape, I.CODA_RATIO)
+        want = REF[f"labels.{shape}.{width}.{ci}"]
+        for row, name in enumerate(("det", "ppk", "spk")):
+            assert np.array_equal(got[row], want[row]), (shape, width, ppks, spks, name)

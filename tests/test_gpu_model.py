@@ -10,6 +10,7 @@ import os
 import pytest
 import torch
 
+from oracle import fixtures
 from oracle import seist_ref as R
 from seist_b200.models import BCELoss, HuberLoss, create_model
 
@@ -18,7 +19,7 @@ ZERO = dict(path_drop_rate=0, attn_drop_rate=0, key_drop_rate=0, mlp_drop_rate=0
 
 
 def _load(name):
-    g = torch.load(os.path.join(GOLD, f"{name}.pt"))
+    g = fixtures.load(GOLD, name)
     m = create_model(name, in_channels=3, in_samples=g["x"].shape[-1])
     m.load_state_dict(g["state_dict"], strict=True)
     return g, m.cuda()
